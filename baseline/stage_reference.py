@@ -5,7 +5,7 @@ The reference has no setup.py / pyproject.toml (it is used from its source tree,
 two importable packages `pytracking/` and `ltr/` byte for byte; nothing is edited.  `baseline/ref_env.py` then puts
 baseline/_ref on sys.path and installs the out-of-tree compatibility shims (SURVEY.md 8(c)).
 
-    python baseline/stage_reference.py            # idempotent; run by __graft_entry__.build() when /root/reference exists
+    PYTRACKING_REFERENCE=<pytracking checkout> python baseline/stage_reference.py        # idempotent
 """
 import hashlib
 import os

@@ -72,6 +72,9 @@ def parse():
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--precision", type=int, default=0)
     ap.add_argument("--no-baselines", action="store_true", help="skip cpu_baseline / torch_cuda_baseline (profiling runs)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step of each leg returned as DIR/<name>.npy (dimp50 --impl b200 only): "
+                         "target_bbox, scores and filter of the device-resident leg, e2e_target_bbox of the host-buffer leg")
     ap.add_argument("--config", default="dimp50", choices=["dimp50", "prdimp50", "atom", "tomp101", "eco", "dimp_simple"],
                     help="dimp50 = BASELINE configs[1] (the metric of record, native whole-frame tracker); the others time the UNMODIFIED "
                          "reference tracker of BASELINE configs[2] / [0] / [3] above the engine (plugin.install()) against the same tracker "
@@ -301,6 +304,9 @@ def run_b200(args, rank, world, local_rank):
     torch.cuda.synchronize(); barrier()
     dev_ms = e0.elapsed_time(e1)
     launches = _lib.lib().b200trk_launch_count() - launches0
+    # what the last timed track_device returned, read back after the timed region
+    outputs = {"target_bbox": np.array(trk.info.bbox, dtype=np.float64), "scores": trk.engine.scores.float().cpu().numpy(),
+               "filter": trk.engine.filter.float().cpu().numpy()}
     f += W + K
     del dev_frames
 
@@ -318,6 +324,11 @@ def run_b200(args, rank, world, local_rank):
     torch.cuda.synchronize()
     host_ms = (time.perf_counter() - t0) * 1e3
     gc.enable()
+    outputs["e2e_target_bbox"] = np.array(boxes[-1], dtype=np.float64)
+    if args.dump_outputs and rank == 0:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in outputs.items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
     barrier()
     clocks = sampler.finish() if sampler else None
 
@@ -576,6 +587,8 @@ def run_other(args, rank, world, local_rank):
 
 def main():
     args = parse()
+    if args.dump_outputs and (args.config != "dimp50" or args.impl != "b200"):
+        sys.exit("--dump-outputs: only the dimp50 workload of --impl b200 has outputs to write")
     world = int(os.environ.get("WORLD_SIZE", "1"))
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

@@ -104,52 +104,22 @@ def test_localize_kernel_source_matches_recorded_reference_trajectories(emul):
 
 
 def test_localize_kernel_source_matches_reference_code_on_random_maps(emul):
-    from baseline import ref_env
-    if not ref_env.reference_available():
-        pytest.skip("reference tree not staged (baseline/_ref)")
-    from oracle import ref_shims
-    ref_shims.install(prroi_cpu=False)
-    from pytracking.tracker.dimp.dimp import DiMP
-    from pytracking.utils import TrackerParams
+    """Against the reference `DiMP.localize_target` on seeded random maps (recorded by oracle/gen_localize_golden.py)."""
+    from oracle.gen_localize_golden import cases
     from pytracking_b200.tracker import FLAGS
-    g = torch.Generator().manual_seed(0)
+    d = np.load(os.path.join(GOLDEN, "localize_random.npz"))
+    img_support_sz, out_sz = torch.Tensor([288, 288]), torch.Tensor([18, 18])
     seen = set()
-    for trial in range(200):
-        adv = trial % 10 != 9
-        S = 1 + trial % 3
-        kw = dict(advanced_localization=adv, target_not_found_threshold=0.2, uncertain_threshold=0.25 if trial % 4 == 0 else -float("inf"),
-                  hard_sample_threshold=0.3 if trial % 5 == 0 else -float("inf"), distractor_threshold=0.8, hard_negative_threshold=0.5,
-                  dispalcement_scale=0.3 + 0.5 * (trial % 2))
+    for trial, (kw, scores, target_sz, sample_pos, sample_scales, pos) in enumerate(cases(200)):
         params = _params(**kw)
-        scores = 0.1 * torch.rand(S, 19, 19, generator=g)
-        for s in range(S):
-            for _ in range(1 + trial % 3):               # a few peaks of comparable height
-                r, c = [int(v) for v in torch.randint(0, 19, (2,), generator=g)]
-                scores[s, r, c] = 0.15 + 0.6 * float(torch.rand(1, generator=g))
-        if trial % 7 == 0:                               # exact ties: the arg-max order must follow dcf.max2d
-            scores[0, 3, 11] = scores[0, 12, 4] = scores.max() + 0.1
-        trk = DiMP.__new__(DiMP)
-        p = TrackerParams()
-        for k, v in kw.items():
-            setattr(p, k, v)
-        p.target_neighborhood_scale = 2.2
-        trk.params = p
-        trk.output_window = None
-        trk.kernel_size = torch.Tensor([4, 4])
-        trk.img_support_sz = torch.Tensor([288, 288])
-        trk.target_sz = torch.Tensor([60, 80]) * (0.5 + float(torch.rand(1, generator=g)))
-        sample_scales = 1.0 + 0.5 * torch.rand(S, generator=g)
-        sample_pos = torch.Tensor([[240, 320]]).repeat(S, 1) + torch.rand(S, 2, generator=g)
-        trk.pos = sample_pos[0] + 40 * (torch.rand(2, generator=g) - 0.5)
-        tv, scale_ind, _, flag = trk.localize_target(scores.clone().unsqueeze(1), sample_pos, sample_scales)
-        out_sz = torch.Tensor([18, 18])
-        neigh = [(2.2 * (trk.target_sz / sample_scales[s]) * (out_sz / trk.img_support_sz)).numpy() for s in range(S)]
-        pv = [((trk.pos - sample_pos[s]) / ((trk.img_support_sz / out_sz) * sample_scales[s])).numpy() for s in range(S)]
+        S = scores.shape[0]
+        neigh = [(2.2 * (target_sz / sample_scales[s]) * (out_sz / img_support_sz)).numpy() for s in range(S)]
+        pv = [((pos - sample_pos[s]) / ((img_support_sz / out_sz) * sample_scales[s])).numpy() for s in range(S)]
         out = _run_localize(emul, scores, params, neigh, pv)
-        assert FLAGS[out.flag] == flag, (trial, FLAGS[out.flag], flag)
-        assert out.scale_ind == int(scale_ind)
+        assert out.flag == d["flag"][trial], (trial, FLAGS[out.flag], FLAGS[d["flag"][trial]])
+        assert out.scale_ind == d["scale_ind"][trial]
         cell = (out.r2, out.c2) if out.use_second else (out.r1, out.c1)
-        mine = (torch.Tensor(cell) - 9) * (trk.img_support_sz / out_sz) * sample_scales[scale_ind]
-        assert torch.equal(mine, tv), (trial, mine, tv)
-        seen.add((flag, out.use_second))
+        mine = (torch.Tensor(cell) - 9) * (img_support_sz / out_sz) * sample_scales[out.scale_ind]
+        assert torch.equal(mine, torch.from_numpy(d["tv"][trial])), (trial, mine, d["tv"][trial])
+        seen.add((FLAGS[out.flag], out.use_second))
     assert {("normal", 0), ("hard_negative", 0), ("hard_negative", 1), ("uncertain", 0), ("not_found", 0), (None, 0)} <= seen, seen

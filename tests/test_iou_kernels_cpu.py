@@ -1,7 +1,8 @@
 """IoUNet box refinement (SURVEY 8 row f1) executed ON THE CPU: the kernels of csrc/iou_refine_kernels.cuh + csrc/prroi_kernels.cuh -- the
 same source files the CUDA build compiles (`cuobjdump -sass` identical before and after they moved into headers) -- built as host code under
 tests/cpu_emul/cuda_shim.h and run in the launch sequence of `b200trk_iou_predict` / `b200trk_iou_refine` (csrc/iou_refine.cu), against
-the UNMODIFIED reference: `AtomIoUNet.predict_iou` with torch autograd for the box gradient (ltr/models/bbreg/atom_iou_net.py:96-136) and
+what the UNMODIFIED reference computed for the same seeded weights and inputs (tests/golden/iou.npz, oracle/gen_iou_golden.py):
+`AtomIoUNet.predict_iou` with torch autograd for the box gradient (ltr/models/bbreg/atom_iou_net.py:96-136) and
 `DiMP.optimize_boxes_default / _relative` (pytracking/tracker/dimp/dimp.py:725-793), PrRoIPool from the oracle's CPU restatement.
 CPU-tier counterparts of tests/test_iou_gpu.py."""
 import ctypes as C
@@ -13,9 +14,8 @@ import numpy as np
 import pytest
 import torch
 
-from baseline import ref_env
+from oracle import gen_iou_golden as G
 
-pytestmark = pytest.mark.skipif(not ref_env.reference_available(), reason="reference tree not staged (baseline/_ref)")
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
@@ -30,20 +30,13 @@ def emul(tmp_path_factory):
 
 
 @pytest.fixture(scope="module")
-def net():
-    from oracle import ref_shims
-    ref_shims.install()
-    from baseline import ref_tracker
-    n = ref_tracker.build_dimp_net("resnet50", seed=0)
-    g = torch.Generator().manual_seed(5)
-    for m in n.bb_regressor.modules():                       # non-trivial BN statistics, as in tests/test_iou_gpu.py
-        if isinstance(m, (torch.nn.BatchNorm2d, torch.nn.BatchNorm1d)):
-            m.running_mean.copy_(0.05 * torch.randn(m.running_mean.shape, generator=g))
-            m.running_var.copy_(0.7 + 0.6 * torch.rand(m.running_var.shape, generator=g))
-            m.bias.data.copy_(0.05 * torch.randn(m.bias.shape, generator=g))
-    with torch.no_grad():
-        n.bb_regressor.iou_predictor.weight.mul_(20.0)       # box gradients of O(1e-2): the refinement loops move boxes by pixels
-    return n
+def sd():
+    return G.make_iou_state_dict()
+
+
+@pytest.fixture(scope="module")
+def gold():
+    return np.load(os.path.join(ROOT, "tests", "golden", "iou.npz"))
 
 
 def _rel(a, b):
@@ -51,19 +44,9 @@ def _rel(a, b):
     return float((a - b).abs().max() / (b.abs().max() + 1e-30))
 
 
-def _inputs(seed, R):
-    g = torch.Generator().manual_seed(seed)
-    f3 = torch.relu(torch.randn(1, 256, 36, 36, generator=g))
-    f4 = torch.relu(torch.randn(1, 256, 18, 18, generator=g))
-    mod = [torch.randn(1, 256, 1, 1, generator=g).abs(), torch.randn(1, 256, 1, 1, generator=g).abs()]
-    c = torch.tensor([120.0, 130.0]) + 30 * (torch.rand(R, 2, generator=g) - 0.5)
-    sz = torch.tensor([70.0, 55.0]) * (0.6 + 0.8 * torch.rand(R, 2, generator=g))
-    return mod, [f3, f4], torch.cat([c - sz / 2, sz], 1).reshape(1, R, 4)
-
-
-def _run(emul, net, mod, feat, boxes, num_iter=0, step=1.0, decay=1.0, relative=False, want_grad=True):
+def _run(emul, sd, mod, feat, boxes, num_iter=0, step=1.0, decay=1.0, relative=False, want_grad=True):
     from pytracking_b200 import _lib
-    sd, keep = net.state_dict(), []
+    keep = []
 
     def hp(key):
         t = sd["bb_regressor." + key].detach().float().contiguous()
@@ -91,34 +74,21 @@ def _run(emul, net, mod, feat, boxes, num_iter=0, step=1.0, decay=1.0, relative=
     return iou, grad, bx
 
 
-@pytest.mark.parametrize("seed,R", [(0, 10), (1, 1), (2, 16)])
-def test_predict_iou_and_box_gradient_kernel_sources_vs_reference_autograd(emul, net, seed, R):
-    mod, feat, boxes = _inputs(seed, R)
-    bb = boxes.clone().requires_grad_(True)
-    ref = net.bb_regressor.predict_iou(mod, feat, bb)                # dimp.py:737-742: predict_iou + backward
-    ref.backward(gradient=torch.ones_like(ref))
-    iou, grad, _ = _run(emul, net, mod, feat, boxes)
-    assert _rel(iou, ref.reshape(-1)) < 1e-4 and _rel(grad, bb.grad.reshape(-1, 4)) < 1e-4, (_rel(iou, ref.reshape(-1)), _rel(grad, bb.grad.reshape(-1, 4)))
+@pytest.mark.parametrize("seed,R", G.PREDICT)
+def test_predict_iou_and_box_gradient_kernel_sources_vs_reference_autograd(emul, sd, gold, seed, R):
+    mod, feat, boxes = G.inputs(seed, R)
+    ref_iou, ref_grad = torch.from_numpy(gold["iou_%d" % seed]), torch.from_numpy(gold["grad_%d" % seed])
+    iou, grad, _ = _run(emul, sd, mod, feat, boxes)
+    assert _rel(iou, ref_iou) < 1e-4 and _rel(grad, ref_grad) < 1e-4, (_rel(iou, ref_iou), _rel(grad, ref_grad))
 
 
 @pytest.mark.parametrize("relative", [False, True])
-def test_refinement_loop_kernel_sources_vs_reference_optimize_boxes(emul, net, relative):
-    from pytracking.libs import TensorList
-    from pytracking.tracker.dimp.dimp import DiMP
-    from pytracking.utils import TrackerParams
-    mod, feat, boxes = _inputs(7, 10)
-    p = TrackerParams()
-    p.device = "cpu"
-    p.box_refinement_iter = 4 if relative else 3            # the tracker uses 10 / 5 (tests/test_iou_gpu.py does too); fewer here for time
-    p.box_refinement_step_length = 5e-3 if relative else 1
-    p.box_refinement_step_decay = 1
-    p.box_refinement_space = "relative" if relative else "default"
-    trk = DiMP.__new__(DiMP)
-    trk.params = p
-    trk.net = type("N", (), {"bb_regressor": net.bb_regressor})()
-    trk.iou_modulation = TensorList(mod)
-    ref_boxes, ref_iou = trk.optimize_boxes(TensorList(feat), boxes.reshape(-1, 4).clone())        # the reference loop (autograd)
-    iou, _, b = _run(emul, net, mod, feat, boxes, p.box_refinement_iter, p.box_refinement_step_length, p.box_refinement_step_decay, relative)
+def test_refinement_loop_kernel_sources_vs_reference_optimize_boxes(emul, sd, gold, relative):
+    tag = "cpu_relative" if relative else "cpu_default"   # the tracker uses 10 / 5 iterations (tests/test_iou_gpu.py does too); fewer here for time
+    n_iter, step, _ = G.REFINE[tag]
+    mod, feat, boxes = G.inputs(G.REFINE_SEED, G.REFINE_R)
+    ref_boxes, ref_iou = torch.from_numpy(gold["boxes_" + tag]), torch.from_numpy(gold["iou_" + tag])
+    iou, _, b = _run(emul, sd, mod, feat, boxes, n_iter, step, 1.0, relative)
     assert _rel(b, ref_boxes) < 1e-4 and float((b - ref_boxes).abs().max()) < 2e-2, (_rel(b, ref_boxes), float((b - ref_boxes).abs().max()))
     assert _rel(iou, ref_iou) < 1e-3
     assert float((ref_boxes - boxes.reshape(-1, 4)).abs().max()) > 0.5                              # the loop really moved the boxes
